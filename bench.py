@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: consensus rounds/sec of DiNNO on the dist_mnist_PAPER config.
 
-    python bench.py --gpus N --steps K --warmup W [--impl ours|reference|nccl] [--dtype fp64|fp32]
+    python bench.py --gpus N --steps K --warmup W [--impl ours|reference|nccl] [--dtype fp64|fp32] [--dump-outputs DIR]
     (N > 1: launched by the driver through torch.distributed.run, one rank per GPU)
 
 Config (reference: experiments/dist_mnist_PAPER.yaml problem1): MNISTConvNet(3,5,64),
@@ -35,7 +35,7 @@ reference = the same stock classes under torch.set_default_dtype(float32)).
   ring / complete (NVLS) / random graph x DiNNO / DSGD / DSGT, every edge crosses NVLink.
 * ``extra.multi_gpu_selfcheck`` — (N > 1, untimed) the distributed run's parameters after a few
   rounds against a single-process recomputation on rank 0.
-* ``--impl reference`` — the unmodified reference (baseline/_ref) through its own public API
+* ``--impl reference`` — the unmodified reference (oracle/_ref, installed by ``build()``) through its own public API
   (DistMNISTProblem + DiNNO(...).train(profiler=hook)), all nodes on one device.
 * ``--impl nccl`` — one-rank-per-GPU PyTorch + NCCL re-expression (batched cuDNN/cuBLAS
   forward/backward of all local nodes, all_gather of the parameter rows, torch elementwise
@@ -47,7 +47,6 @@ import argparse
 import json
 import os
 import statistics
-import subprocess
 import sys
 import threading
 import time
@@ -64,6 +63,7 @@ PITS = 2
 SAMPLES_PER_NODE = 22000          # 10 nodes x 22000 x 784 B = 172 MB of uint8 rows per GPU (> 126 MB L2)
 REF_SAMPLES_PER_NODE = 6000       # the paper's 60000 / 10 (the reference streams from host memory anyway)
 PAPER_ROUNDS = 2000
+DUMP_MAX_BYTES = 64 << 20
 METRIC = "consensus node-rounds/sec (DiNNO, dist_mnist_PAPER; rounds/sec x graph nodes)"
 
 
@@ -267,8 +267,29 @@ def _cycle(n):
     return nx.cycle_graph(n) if n > 2 else nx.path_graph(n)
 
 
-def measure_headline(h, ctx, args, dtype, sampler=None, probe=False):
-    """value (resident/staged shards) + e2e (host-fed) of the headline config at ``dtype``."""
+def dump_outputs(out_dir, ctx, pr, opt):
+    """Write what the timed ``run_rounds(K)`` hands its caller after the last timed round, one row per graph node:
+    ``theta`` (parameters, ``parameters_to_vector`` order), ``duals`` (DiNNO dual variables) and ``losses`` (minibatch
+    loss of the round's last primal step).  Above DUMP_MAX_BYTES, theta and duals keep a fixed seeded sample of columns."""
+    import numpy as np
+    arrays = {"theta": pr.arena.compact(pr.gather_rows(pr.arena.theta)), "duals": pr.arena.compact(pr.gather_rows(opt.duals)),
+              "losses": pr.gather_rows(pr.fused.loss_part.sum(1))}
+    if not ctx.is_main:
+        return
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    n = arrays["theta"].shape[1]
+    keep = int((DUMP_MAX_BYTES - arrays["losses"].nbytes) * n // (arrays["theta"].nbytes + arrays["duals"].nbytes))
+    if keep < n:
+        cols = np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+        arrays["theta"], arrays["duals"] = arrays["theta"][:, cols], arrays["duals"][:, cols]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure_headline(h, ctx, args, dtype, sampler=None, probe=False, dump_dir=None):
+    """value (resident/staged shards) + e2e (host-fed) of the headline config at ``dtype``; with ``dump_dir`` the
+    outputs of the last timed round are written there (``dump_outputs``)."""
     import torch
     from nn_distributed_training_b200.optimizers import DiNNO
 
@@ -281,6 +302,8 @@ def measure_headline(h, ctx, args, dtype, sampler=None, probe=False):
     opt = DiNNO(pr, dev, pr.conf["optimizer_config"])
     opt.run_rounds(W)                     # warm-up (captures + runs its own graph)
     ms, _ = h.time_rounds(opt, K, sampler)
+    if dump_dir:
+        dump_outputs(dump_dir, ctx, pr, opt)
     prog = opt._program
     out = {"ms_per_step": ms / K, "value": n_nodes * K / (ms / 1e3), "launches": K * prog.launches_per_round(),
            "pipeline": prog.pipeline, "symm": prog.eng.pub_buf.how, "flags": prog.eng.flag_mode,
@@ -416,7 +439,7 @@ def run_ours(args):
     h = Harness(ctx)
     sampler = ClockSampler(dev.index or 0)
     sampler.start()                       # thread + NVML handle exist before any barrier of a timed region
-    main = measure_headline(h, ctx, args, args.dtype, sampler, probe=args.extras)
+    main = measure_headline(h, ctx, args, args.dtype, sampler, probe=args.extras, dump_dir=args.dump_outputs)
     clocks = sampler.stop()
     extra = {"top1_after_rounds": main["top1_after_rounds"], "rounds_done": main["rounds_done"]}
     if "fixed_cost_probe" in main:
@@ -472,17 +495,15 @@ def run_nccl_baseline(args):
 
 # --------------------------------------------------------------- reference ----
 def ensure_reference():
-    ref = os.path.join(ROOT, "baseline", "_ref")
-    if not os.path.isdir(os.path.join(ref, "optimizers")):
-        subprocess.run(["bash", os.path.join(ROOT, "baseline", "install_reference.sh")],
-                       stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    """The unmodified reference tree that ``build()`` installed (oracle/install_reference.py), or None."""
+    ref = os.path.join(ROOT, "oracle", "_ref")
     return ref if os.path.isdir(os.path.join(ref, "optimizers")) else None
 
 
 def run_reference(args):
     ref = ensure_reference()
     if ref is None:
-        print(json.dumps({"impl": "reference", "unavailable": "baseline/_ref missing and /root/reference not mounted"}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref missing: build() installs the reference there from a checkout of it"}))
         return
     import torch
     import torch.distributed as dist
@@ -584,13 +605,19 @@ def _reference_rank0(args, ref, dtype, budget_s):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed rounds; --impl reference times at most REF_MAX_SECONDS of rounds (at its measured rate "
+                         "per node-round) and reports the rounds it timed as steps, the requested ones as steps_requested")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "nccl"])
     ap.add_argument("--dtype", default=os.environ.get("NNDT_BENCH_DTYPE", "fp64"), choices=["fp64", "fp32"])
     ap.add_argument("--no-extras", dest="extras", action="store_false",
                     help="headline only: skip the other-precision run, the one-node-per-GPU sweep, the self-check and the probe")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed round as DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is implemented for --impl ours")
     if args.impl == "reference":
         if "--steps" not in " ".join(sys.argv):
             args.steps = 100

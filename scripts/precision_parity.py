@@ -3,7 +3,7 @@ NON-separable synthetic set, identical data / seeds / sampler:
 
   * ours fp64 fused  vs  ours fp32 fused: parameter-trajectory distance ||theta32 - theta64|| / ||theta64|| per evaluation
     point, validation accuracy / loss curves of both;
-  * the unmodified reference (baseline/_ref, float64, its own DataLoader shuffling) on the same shards: accuracy / loss
+  * the unmodified reference (oracle/_ref, float64, its own DataLoader shuffling) on the same shards: accuracy / loss
     curve next to ours (different minibatch order, so curves agree statistically, not point-wise).
 
     python scripts/precision_parity.py [--rounds 2000] [--algs dinno,dsgt,dsgd] [--ref-algs dinno] [--out profiles/precision_parity.md]

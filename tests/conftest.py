@@ -7,8 +7,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE = "/root/reference"
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
@@ -25,26 +23,3 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords or "multigpu" in item.keywords:
             item.add_marker(skip)
-
-
-@pytest.fixture(scope="session")
-def reference():
-    """Import handle on the unmodified reference tree (oracle for semantics)."""
-    if not os.path.isdir(os.path.join(REFERENCE, "optimizers")):
-        pytest.skip("reference tree not mounted")
-    import importlib
-    import types
-
-    sys.path.insert(0, REFERENCE)
-    try:
-        ns = types.SimpleNamespace(
-            dinno=importlib.import_module("optimizers.dinno"),
-            dsgd=importlib.import_module("optimizers.dsgd"),
-            dsgt=importlib.import_module("optimizers.dsgt"),
-            mnist_problem=importlib.import_module("problems.dist_mnist_problem"),
-            mnist_model=importlib.import_module("models.mnist_conv_nn"),
-            graphs=importlib.import_module("utils.graph_generation"),
-        )
-    finally:
-        sys.path.remove(REFERENCE)
-    return ns

@@ -43,7 +43,7 @@ def test_reference_arm_runs_the_unmodified_reference(monkeypatch):
     import bench
     ref = bench.ensure_reference()
     if ref is None:
-        pytest.skip("reference tree not available")
+        pytest.skip("oracle/_ref not installed (build() installs it from a checkout of the reference)")
     monkeypatch.setattr(bench, "StepTimer", _CpuTimer)
     monkeypatch.setattr(bench, "ClockSampler", _NoClocks)
     monkeypatch.setattr(bench, "REF_SAMPLES_PER_NODE", 128)
@@ -67,6 +67,35 @@ def test_reference_arm_runs_the_unmodified_reference(monkeypatch):
     assert line["e2e"]["h2d_bytes_per_step"] > 0
     # both arms print the same config dict (the driver compares them)
     assert line["config"] == bench.headline_config(1)
+
+
+def test_dump_outputs_writes_compact_rows_within_the_size_cap(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    from nn_distributed_training_b200.models import MNISTConvNet
+    from nn_distributed_training_b200.parallel.arena import FlatLayout, NodeArena
+    from nn_distributed_training_b200.parallel.context import DistContext
+
+    arena = NodeArena(FlatLayout.from_module(MNISTConvNet(3, 5, 64)), 3, "cpu", torch.float64)
+    arena.theta.normal_()
+    pr = types.SimpleNamespace(arena=arena, gather_rows=lambda t: t,
+                               fused=types.SimpleNamespace(loss_part=torch.rand(3, 2)))
+    opt = types.SimpleNamespace(duals=arena.theta * 2)
+    bench.dump_outputs(str(tmp_path / "full"), DistContext.single(), pr, opt)
+    got = {n: np.load(tmp_path / "full" / f"{n}.npy") for n in ("theta", "duals", "losses")}
+    np.testing.assert_array_equal(got["theta"], arena.compact(arena.theta).numpy())
+    np.testing.assert_array_equal(got["duals"], 2 * got["theta"])
+    np.testing.assert_array_equal(got["losses"], pr.fused.loss_part.sum(1).numpy())
+    assert got["theta"].dtype == np.float64 and got["losses"].dtype == np.float32
+
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 200_000)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), DistContext.single(), pr, opt)
+    small = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("theta", "duals", "losses")}
+    assert sum(a.nbytes for a in small.values()) <= 200_000 and 0 < small["theta"].shape[1] < got["theta"].shape[1]
+    np.testing.assert_array_equal(small["duals"], 2 * small["theta"])
+    np.testing.assert_array_equal(small["theta"], np.load(tmp_path / "b" / "theta.npy"))      # the same sample every run
 
 
 def test_reference_arm_caps_the_timed_region():

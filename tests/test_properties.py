@@ -1,5 +1,6 @@
 """Property tests of topology, sampling and the consensus updates (SURVEY §4 item 4)."""
 import copy
+import os
 
 import networkx as nx
 import numpy as np
@@ -27,9 +28,20 @@ def test_metropolis_is_symmetric_doubly_stochastic(graph):
     assert ((W > 0) & ~torch.eye(len(graph), dtype=torch.bool) == A).all()
 
 
-def test_metropolis_matches_reference(reference):
-    for g in [nx.cycle_graph(10), nx.wheel_graph(7), nx.erdos_renyi_graph(12, 0.4, seed=1)]:
-        torch.testing.assert_close(gg.get_metropolis(g, dtype=torch.float64), reference.graphs.get_metropolis(g).double())
+def metropolis_graphs():
+    return [nx.cycle_graph(10), nx.wheel_graph(7), nx.erdos_renyi_graph(12, 0.4, seed=1)]
+
+
+@pytest.fixture(scope="module")
+def golden():
+    """The reference's own outputs on the inputs built here (written by oracle/make_golden.py)."""
+    with np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_properties.npz")) as z:
+        return dict(z)
+
+
+def test_metropolis_matches_reference(golden):
+    for i, g in enumerate(metropolis_graphs()):
+        torch.testing.assert_close(gg.get_metropolis(g, dtype=torch.float64), torch.as_tensor(golden[f"metropolis/{i}"]))
 
 
 def test_complete_graph_metropolis_is_uniform():
@@ -224,27 +236,27 @@ def test_link_drop_fault_injection_changes_graph_and_training_survives():
     assert pr._graph_round == 5
 
 
-def test_lidar_matches_reference_scans():
+def lidar_inputs():
+    """The reference's floor plan and first tight path (shipped unchanged under floorplans/32_data)."""
+    d = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "floorplans", "32_data")
+    return os.path.join(d, "floor_img.png"), np.load(os.path.join(d, "tight_paths", "1.npy"))
+
+
+def lidar_trajectory(interpolate_waypoints, wp, lidar):
+    return interpolate_waypoints(wp[:, 0], wp[:, 1], 1)[::6] * np.array([lidar.nx * 0.5, lidar.ny * 0.5])
+
+
+def test_lidar_matches_reference_scans(golden):
     """Vectorised lidar vs the reference's per-beam Python loops on the reference's own floor plan."""
-    import importlib.util, os
-    ref_py = "/root/reference/floorplans/lidar/lidar.py"
-    img = "/root/reference/floorplans/32_data/floor_img.png"
-    if not (os.path.exists(ref_py) and os.path.exists(img)):
-        pytest.skip("reference floor plan not mounted")
-    spec = importlib.util.spec_from_file_location("reflidar", ref_py)
-    ref = importlib.util.module_from_spec(spec); spec.loader.exec_module(ref)
     from nn_distributed_training_b200.floorplans.lidar import ClippedLidar2D, Lidar2D, interpolate_waypoints
-    args = (img, 12, 0.2, 15, 1.0, 30, 3)
-    mine, theirs = Lidar2D(*args, border_width=30), ref.Lidar2D(*args, border_width=30)
-    wp = np.load("/root/reference/floorplans/32_data/tight_paths/1.npy")
-    np.testing.assert_allclose(interpolate_waypoints(wp[:, 0], wp[:, 1], 3), ref.interpolate_waypoints(wp[:, 0], wp[:, 1], 3))
-    traj = interpolate_waypoints(wp[:, 0], wp[:, 1], 1)[::6] * np.array([mine.nx * 0.5, mine.ny * 0.5])
-    a = mine.scan_batch(traj)
-    b = np.stack([theirs.scan(p.reshape(1, 2)) for p in traj])
-    np.testing.assert_allclose(a, b, rtol=1e-9, atol=1e-9)
-    cm, ct = ClippedLidar2D(img, 12, 0.2, 15, border_width=30), ref.ClippedLidar2D(img, 12, 0.2, 15, border_width=30)
-    for p in traj[:4]:
-        np.testing.assert_allclose(cm.scan(p.reshape(1, 2)), ct.scan(p.reshape(1, 2)), rtol=1e-9, atol=1e-9)
+    img, wp = lidar_inputs()
+    mine = Lidar2D(img, 12, 0.2, 15, 1.0, 30, 3, border_width=30)
+    np.testing.assert_allclose(interpolate_waypoints(wp[:, 0], wp[:, 1], 3), golden["lidar/interp3"])
+    traj = lidar_trajectory(interpolate_waypoints, wp, mine)
+    np.testing.assert_allclose(mine.scan_batch(traj), golden["lidar/scans"], rtol=1e-9, atol=1e-9)
+    cm = ClippedLidar2D(img, 12, 0.2, 15, border_width=30)
+    for i, p in enumerate(traj[:4]):
+        np.testing.assert_allclose(cm.scan(p.reshape(1, 2)), golden[f"lidar/clipped/{i}"], rtol=1e-9, atol=1e-9)
 
 
 def test_round_timer_as_profiler_hook():
