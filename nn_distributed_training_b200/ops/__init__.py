@@ -59,10 +59,13 @@ def mnist_kernel_supports(spec, batch_size: int, dtype=None) -> bool:
     return 1 <= spec.num_filters <= 8 and spec.kernel_size in (3, 5) and 1 <= spec.linear_width <= 128
 
 
-def mlp_kernel_supports(spec, base_loss) -> bool:
-    """Shapes/losses the tcgen05 MLP kernel (csrc/mlp_tc.cu) is instantiated for."""
+def mlp_kernel_supports(spec, base_loss, dtype=None) -> bool:
+    """Shapes/losses/dtypes the implicit-density MLP kernels are instantiated for: csrc/mlp_tc.cu (tcgen05) in fp32,
+    csrc/mlp_f64.cu in fp64, the same network family in both."""
+    import torch
+
     try:
         from .mlp_fused import supports
     except Exception:  # noqa: BLE001
         return False
-    return supports(spec, base_loss)
+    return supports(spec, base_loss, torch.float32 if dtype is None else dtype)

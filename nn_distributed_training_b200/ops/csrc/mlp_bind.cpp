@@ -1,4 +1,4 @@
-// Bindings of the tcgen05 MLP kernels (mlp_tc.cu).
+// Bindings of the implicit-density MLP kernels (mlp_tc.cu: float, mlp_f64.cu: double), the lidar kernels and the generic MLP kernels.
 #include <torch/extension.h>
 #include <ATen/cuda/CUDAContext.h>
 #include <pybind11/pybind11.h>
@@ -22,28 +22,39 @@ void check(cudaError_t e, const char* what) {
   if (e != cudaSuccess) throw std::runtime_error(std::string(what) + ": " + cudaGetErrorString(e));
 }
 
-struct MlpOp {
-  mlp::Args a{};
+// T = float: tcgen05 kernels (mlp_tc.cu); T = double: fp64 kernels (mlp_f64.cu).  Every pointer, and `scale`, is T.
+template <typename T>
+struct MlpOpT {
+  mlp::ArgsT<T> a{};
   int fwd_ctas = 1, train_ctas = 1;
-  explicit MlpOp(const py::dict& d) { update(d); }
+  explicit MlpOpT(const py::dict& d) { update(d); }
   void update(const py::dict& d) {
-    a.theta = ptr<const float>(d, "theta"); a.n_pad = geti(d, "n_pad"); a.L = geti(d, "L");
+    a.theta = ptr<const T>(d, "theta"); a.n_pad = geti(d, "n_pad"); a.L = geti(d, "L");
     auto off = d["off"].cast<std::vector<int>>();
     for (int i = 0; i < 10; ++i) a.off[i] = off.at(i);
     a.d_in = geti(d, "d_in"); a.h1 = geti(d, "h1");
     a.first_act = geti(d, "first_act"); a.last_act = geti(d, "last_act"); a.loss = geti(d, "loss");
-    a.scale = (float)getf(d, "scale", 1.0);
-    a.x = ptr<const float>(d, "x"); a.y = ptr<const float>(d, "y");
-    a.n_rows = geti(d, "n_rows"); a.out = ptr<float>(d, "out");
+    a.scale = (T)getf(d, "scale", 1.0);
+    a.x = ptr<const T>(d, "x"); a.y = ptr<const T>(d, "y");
+    a.n_rows = geti(d, "n_rows"); a.out = ptr<T>(d, "out");
     a.direct = geti(d, "direct"); a.batch = geti(d, "batch"); a.seed = geti(d, "seed"); a.node0 = geti(d, "node0");
     a.shard_off = ptr<const int>(d, "shard_off"); a.shard_len = ptr<const int>(d, "shard_len");
     a.calls = ptr<const int>(d, "calls"); a.win_table = ptr<const int64_t>(d, "win_table");
-    a.grad_part = ptr<float>(d, "grad_part"); a.loss_part = ptr<float>(d, "loss_part"); a.S = geti(d, "S", 1);
+    a.grad_part = ptr<T>(d, "grad_part"); a.loss_part = ptr<T>(d, "loss_part"); a.S = geti(d, "S", 1);
     fwd_ctas = geti(d, "fwd_ctas", 1); train_ctas = geti(d, "train_ctas", 1);
   }
   void forward() { check(mlp::launch_forward(a, fwd_ctas, at::cuda::getCurrentCUDAStream().stream()), "mlp_forward"); }
   void train() { check(mlp::launch_train(a, train_ctas, at::cuda::getCurrentCUDAStream().stream()), "mlp_train"); }
 };
+
+template <typename T>
+void bind_op(py::module& m, const char* name) {
+  py::class_<MlpOpT<T>>(m, name)
+      .def(py::init<const py::dict&>())
+      .def("update", &MlpOpT<T>::update)
+      .def("forward", &MlpOpT<T>::forward)
+      .def("train", &MlpOpT<T>::train);
+}
 }  // namespace
 
 static lidar::Args lidar_args(const py::dict& d) {
@@ -94,9 +105,6 @@ void bind_mlp(py::module& m) {
     check(lidar::launch_density(lidar_args(d), reinterpret_cast<const double*>(xy), n, reinterpret_cast<double*>(out),
                                 at::cuda::getCurrentCUDAStream().stream()), "lidar_density");
   });
-  py::class_<MlpOp>(m, "MlpOp")
-      .def(py::init<const py::dict&>())
-      .def("update", &MlpOp::update)
-      .def("forward", &MlpOp::forward)
-      .def("train", &MlpOp::train);
+  bind_op<float>(m, "MlpOp");
+  bind_op<double>(m, "MlpOpF64");
 }

@@ -227,9 +227,6 @@ cudaError_t launch_forward(const Args& a, int ctas_per_node, cudaStream_t st) {
 //   [256,384) dW1^T (2 blocks of 128 input features x 64) | [384,416) [dW0 | db0] (2 blocks x 16) |
 //   [416,432) db3 | [432,448) db2 | [448,464) db1   (bias sums live in column DIN of their block)
 // =====================================================================================
-constexpr int kWinMax = 64;                           // max windows per period of the online stream
-constexpr int kWinTableLen = 2 + (kWinMax + 1) + 2 * kWinMax;
-
 template <int H1>
 struct TrainSmem {
   alignas(1024) uint8_t w1[(H1 / 64) * W_SLAB];
@@ -448,14 +445,7 @@ __global__ void __launch_bounds__(NTT, 1) mlp_train_kernel(const Args a) {
         if (a.direct) {
           my_idx = (int)(l * a.batch + t);
         } else if (wt != nullptr) {
-          // sliding window stream (floorplans/lidar/lidar.py:397-424 as index arithmetic)
-          const long long K = wt[0], P = wt[1];
-          const long long d = first_draw + t, q = d / P, r = d - q * P;
-          int w = 0;
-          while (w + 1 < K && wt[2 + w + 1] <= r) ++w;
-          const long long lb = wt[2 + kWinMax + 1 + w], ub = wt[2 + kWinMax + 1 + kWinMax + w];
-          const uint32_t wkey = mix_key((uint32_t)a.seed, (uint32_t)(a.node0 + l), (uint32_t)(q * K + w));
-          my_idx = shard_off + (int)lb + (int)feistel_permute((uint32_t)(r - wt[2 + w]), (uint32_t)(ub - lb), wkey);
+          my_idx = shard_off + window_draw(wt, first_draw + t, (uint32_t)a.seed, (uint32_t)(a.node0 + l));
         } else {
           my_idx = shard_off + (int)feistel_permute(start + t, m, key);
         }

@@ -53,4 +53,21 @@ NNDT_DEVINL BatchLoc locate_batch(uint32_t call, uint32_t m, uint32_t B) {
   return o;
 }
 
+// Online sliding-window stream (floorplans/lidar/lidar.py:397-424 as index arithmetic).  One period of a node's
+// stream is described by the table [K, P, cum[0..kWinMax], lb[kWinMax], ub[kWinMax]] (ops/mlp_fused.py:
+// FusedMLP._window_table): K windows of rows [lb, ub), P draws per period, window w starting at draw cum[w].
+constexpr int kWinMax = 64;
+constexpr int kWinTableLen = 2 + (kWinMax + 1) + 2 * kWinMax;
+
+// shard row of draw d (counted from the start of the stream) of node `node`
+NNDT_DEVINL int window_draw(const long long* wt, long long d, uint32_t seed, uint32_t node) {
+  const long long K = wt[0], P = wt[1];
+  const long long q = d / P, r = d - q * P;
+  int w = 0;
+  while (w + 1 < K && wt[2 + w + 1] <= r) ++w;
+  const long long lb = wt[2 + kWinMax + 1 + w], ub = wt[2 + kWinMax + 1 + kWinMax + w];
+  const uint32_t wkey = mix_key(seed, node, (uint32_t)(q * K + w));
+  return (int)lb + (int)feistel_permute((uint32_t)(r - wt[2 + w]), (uint32_t)(ub - lb), wkey);
+}
+
 }  // namespace nndt

@@ -1,4 +1,5 @@
-"""Python side of the tcgen05 MLP kernels (csrc/mlp_tc.cu)."""
+"""Python side of the implicit-density MLP kernels: float32 on the tcgen05 kernels (csrc/mlp_tc.cu, bf16 operands),
+float64 on the CUDA-core fp64 kernels (csrc/mlp_f64.cu)."""
 from __future__ import annotations
 
 import numpy as np
@@ -19,9 +20,17 @@ def shape_supported(spec: MLPSpec) -> bool:
             and spec.first in FIRST and spec.hidden == "relu" and spec.last in LAST)
 
 
-def supports(spec: MLPSpec, base_loss) -> bool:
-    return (TRAIN_KERNEL_READY and shape_supported(spec) and type(base_loss).__name__ in LOSS
-            and getattr(base_loss, "reduction", "mean") == "mean")
+def supports(spec: MLPSpec, base_loss, dtype=torch.float32) -> bool:
+    """Both arms cover the same network family and losses."""
+    return (TRAIN_KERNEL_READY and dtype in (torch.float32, torch.float64) and shape_supported(spec)
+            and type(base_loss).__name__ in LOSS and getattr(base_loss, "reduction", "mean") == "mean")
+
+
+F64_TILE = 64       # batch rows per tile of the fp64 kernels
+
+
+def _op_class(ext, dtype):
+    return ext.MlpOp if dtype == torch.float32 else ext.MlpOpF64
 
 
 def op_dict(arena, spec: MLPSpec, L: int):
@@ -32,22 +41,26 @@ def op_dict(arena, spec: MLPSpec, L: int):
 
 
 class MlpForward:
-    """Forward-only evaluation of every local node's network on shared inputs ``x [M, d_in]``."""
+    """Forward-only evaluation of every local node's network on shared inputs ``x [M, d_in]``, in the arena's dtype."""
 
     def __init__(self, arena, spec: MLPSpec, L: int, device):
         self.ext = load_ext(required=True)
         self.arena, self.spec, self.L, self.device = arena, spec, L, device
+        self.dtype = arena.dtype
         self.sms = torch.cuda.get_device_properties(device).multi_processor_count
         self._cache = {}
 
     def __call__(self, x: torch.Tensor) -> torch.Tensor:
-        x = x.to(torch.float32).contiguous()
+        x = x.to(self.dtype).contiguous()
         M = x.shape[0]
-        out = torch.empty(self.L, M, dtype=torch.float32, device=self.device)
+        out = torch.empty(self.L, M, dtype=self.dtype, device=self.device)
         d = op_dict(self.arena, self.spec, self.L)
-        ctas = max(1, min(-(-M // 128), max(1, (2 * self.sms) // max(1, self.L))))
+        if self.dtype == torch.float32:
+            ctas = max(1, min(-(-M // 128), max(1, (2 * self.sms) // max(1, self.L))))
+        else:       # one fp64 CTA per SM
+            ctas = max(1, min(-(-M // F64_TILE), self.sms // max(1, self.L)))
         d.update(x=x.data_ptr(), n_rows=M, out=out.data_ptr(), fwd_ctas=ctas)
-        op = self.ext.MlpOp(d)
+        op = _op_class(self.ext, self.dtype)(d)
         op.forward()
         self._keep = (x, out, op)
         return out
@@ -56,7 +69,7 @@ class MlpForward:
 class FusedMLP:
     """Fused training/eval engine of a density problem (FourierNet family) — the analogue of
     ``FusedMnist``: device-resident shards, stateless sampling, per-CTA gradient partials that
-    the consensus update kernel sums."""
+    the consensus update kernel sums.  Shards, partials and outputs are kept in the arena dtype."""
 
     def __init__(self, problem):
         self.pr = problem
@@ -65,18 +78,25 @@ class FusedMLP:
         a, pl = problem.arena, problem.placement
         self.spec = problem.base_model.spec
         self.L, self.n_pad, self.B = pl.L, a.n_pad, problem.train_batch_size
+        self.dtype = a.dtype
         self.sms = torch.cuda.get_device_properties(dev).multi_processor_count
-        tmax = -(-self.B // 128)
-        self.G = max(1, min(self.sms, self.L * tmax))
-        self.S = -(-self.G // self.L) + 1
+        if self.dtype == torch.float32:
+            # static partition of the (node, 128-row tile) items over G CTAs; a node spans at most S of them
+            tmax = -(-self.B // 128)
+            self.G = max(1, min(self.sms, self.L * tmax))
+            self.S = -(-self.G // self.L) + 1
+        else:
+            # grid (S, L), one CTA per SM: CTA s of a node takes its tiles s, s + S, ...
+            self.S = max(1, min(-(-self.B // F64_TILE), self.sms // self.L))
+            self.G = self.S * self.L
         sh = problem.shards
-        self.x = sh.x.to(torch.float32).contiguous()
-        self.y = sh.y.to(torch.float32).contiguous()
+        self.x = sh.x.to(self.dtype).contiguous()
+        self.y = sh.y.to(self.dtype).contiguous()
         self.shard_off = torch.tensor(sh.offsets[:-1], dtype=torch.int32, device=dev)
         self.shard_len = torch.tensor(sh.sizes, dtype=torch.int32, device=dev)
         self.calls = torch.zeros(self.L, dtype=torch.int32, device=dev)
-        self.grad_part = torch.zeros(self.L, self.S, self.n_pad, dtype=torch.float32, device=dev)
-        self.loss_part = torch.zeros(self.L, self.S, dtype=torch.float32, device=dev)
+        self.grad_part = torch.zeros(self.L, self.S, self.n_pad, dtype=self.dtype, device=dev)
+        self.loss_part = torch.zeros(self.L, self.S, dtype=self.dtype, device=dev)
         self.win_table = self._window_table()
         d = op_dict(a, self.spec, self.L)
         d.update(win_table=None if self.win_table is None else self.win_table.data_ptr())
@@ -86,7 +106,7 @@ class FusedMLP:
                  calls=self.calls.data_ptr(), grad_part=self.grad_part.data_ptr(),
                  loss_part=self.loss_part.data_ptr(), S=self.S, train_ctas=self.G)
         self.base = d
-        self.train_op = self.ext.MlpOp(d)
+        self.train_op = _op_class(self.ext, self.dtype)(d)
         self._fwd = MlpForward(a, self.spec, self.L, dev)
         self.host_feed = None
 

@@ -72,7 +72,7 @@ class DensityProblemBase(ConsensusProblem):
         if not isinstance(spec, MLPSpec):
             return False
         from ..ops import fused_available, mlp_kernel_supports
-        return self.dtype == torch.float32 and fused_available() and mlp_kernel_supports(spec, self.base_loss)
+        return fused_available() and mlp_kernel_supports(spec, self.base_loss, self.dtype)
 
     def _setup_fused(self):
         from ..ops.mlp_fused import FusedMLP

@@ -107,6 +107,9 @@ configs["dist_online_dense_PAPER.yaml"] = {
         "problem2": online_problem("dsgt", 20000, dsgt(4000, 0.001)),
         "problem3": online_problem("dsgd", 20000, dsgd(4000, 0.001, 0.001)),
     }}
+# the PAPER run with the reference's precision (float64 everywhere, csrc/mlp_f64.cu forward/backward)
+configs["dist_online_dense_PAPER_f64.yaml"] = copy.deepcopy(configs["dist_online_dense_PAPER.yaml"])
+configs["dist_online_dense_PAPER_f64.yaml"]["experiment"].update(name="dist_online_dense_PAPER_f64", dtype="float64")
 configs["dist_online_dense_anim.yaml"] = {
     "experiment": online_exp("dist_online_dense_anim", 15000, False),
     "problem_configs": {"problem1": online_problem(
